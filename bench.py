@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # N>1: launched by torchrun, one rank per GPU
     python bench.py --impl reference ...                     # the CPU implementation of the same path (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/<name>.npy
 
 Prints ONE JSON line (rank 0).  `value` = whole-job frames/s with the batch resident in HBM; `e2e` = the same metric
 through TrainStep.step() with pinned HOST batches (H2D of every input + D2H of the loss inside the timed region).
@@ -125,6 +126,23 @@ def decoder_flops_per_frame(H, C=128):
     return 2 * mac
 
 
+DUMP_SAMPLE = 1 << 21      # entries of the flat parameter / gradient vectors written by --dump-outputs
+
+
+def dump_outputs(d, stepper, loss):
+    """What the caller of the timed train step receives from its last step: the loss, the loss terms and, as the step's effect on
+    the model, the updated parameters and the gradients they were updated with.  The two flat vectors hold ~25.5 M values each
+    at the default workload, so both are written as the same fixed seeded sample of DUMP_SAMPLE indices (sorted)."""
+    os.makedirs(d, exist_ok=True)
+    p, g = stepper.optimizer.flat_param, stepper.optimizer.flat_grad
+    n = p.numel()
+    idx = np.arange(n) if n <= DUMP_SAMPLE else np.sort(np.random.RandomState(0).randint(0, n, size=DUMP_SAMPLE))
+    idx = torch.from_numpy(idx).to(p.device)
+    out = dict(loss=loss, loss_terms=stepper.terms, params_sample=p[idx], grads_sample=g[idx])
+    for name, v in out.items():
+        np.save(os.path.join(d, name + ".npy"), v.detach().float().cpu().numpy())
+
+
 SPANS = ("decoder_fwd", "decoder_bwd", "decoder_wgrad", "loss", "encoders_fwd", "encoders_bwd", "optimizer", "weight_pack")
 
 
@@ -176,6 +194,9 @@ def run_ours(args):
         return float(t.item())
 
     def measure(B, T, H, T_ex, K, W, timing=False, label_Z=0):
+        # dropout masks and VAE noise come from torch's generators, whose default seed changes from process to process: seeded
+        # here, runs with the same arguments compute the same steps
+        torch.manual_seed(1234)
         stepper, P, stats = build_stepper(H, device, world, use_graph=bool(args.graph), label_Z=label_Z)
         dbatch = synth_batch(B, T, T_ex, seed=100 + rank, device=device, label_Z=label_Z)
         graphed = bool(args.graph)
@@ -220,6 +241,8 @@ def run_ours(args):
             ar_ms = max_over_ranks(sum(a.elapsed_time(b) for a, b in stepper.ar_events) / len(stepper.ar_events))
         stepper.ar_events = None
         clocks = sampler.stop() if (rank == 0 and timing) else None
+        if timing and rank == 0 and args.dump_outputs:
+            dump_outputs(args.dump_outputs, stepper, loss)
         if clocks is not None:
             clocks["note"] = "nvidia-smi every 200 ms from the start of 24 untimed warm steps of the same loop through the timed region"
         spans, span_src = {}, None
@@ -494,7 +517,14 @@ if __name__ == "__main__":
     ap.add_argument("--pin", type=int, default=1, help="bind the launch thread to the CPUs of the GPU's NUMA node")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--engine", default="tc", choices=["tc", "fp32", "auto"], help="decoder recurrence engine: tcgen05 bf16 (default) or fp32 SIMT")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32): loss, loss_terms, and a "
+                         "fixed seeded sample of the updated parameters (params_sample) and of their gradients (grads_sample)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA train step (--impl ours)")
     if a.impl == "reference":
         run_reference(a)
     else:

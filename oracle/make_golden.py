@@ -178,6 +178,8 @@ def main(only=None):
                 write_generate_golden()
             elif tag == "pose_post":
                 write_pose_post_golden()
+            elif tag in REFERENCE_IO:
+                REFERENCE_IO[tag]()
             else:
                 write_train_golden(tag)
         return
@@ -207,6 +209,8 @@ def main(only=None):
     write_v1_golden()
     write_pose_post_golden()
     write_generate_golden()
+    for fn in REFERENCE_IO.values():
+        fn()
 
     # ---- RAdam trajectory (optimizers.py), 8 steps crossing the N_sma>=5 switch (step 6)
     ref_shim.install()
@@ -304,6 +308,112 @@ def write_generate_golden(H=256):
     print("generate_e2e golden:", {k: getattr(v, "shape", v) for k, v in out.items()})
 
 
+def write_mel_clip_golden():
+    """preprocess_audio (data_pipeline.py:33) on a 1.5 s clip resampled to 90 frames at 60 fps."""
+    pa = ref_shim.ref_preprocess_audio()
+    wav = synth.make_waveforms(1, 24000, seed=3)[0]
+    feat = pa(wav, 60, 90, audio_params(200), ["mel_spec", "energy"])
+    np.savez_compressed(os.path.join(GOLD, "mel_clip90.npz"), wav_seed=3, n_samples=24000, feat=feat)
+    print("mel_clip90 golden written")
+
+
+DATASET_CASES = [(64, 128), (100, 256), (64, 64)]      # (window, example_window_length)
+
+
+def write_dataset_golden():
+    """The reference SGDataset (dataset.py:9-204) on tests/_fixtures.write_processed_data: for 42 seeded windows per case, the
+    window rows, range index and a fingerprint of each of the 11 tensors __getitem__ returns; and the one-hot labels of every
+    window."""
+    import tempfile
+    from tests import _fixtures as fx
+    ref_shim.install()
+    import dataset as ref_dataset
+    ddef, dproc = fx.write_processed_data(tempfile.mkdtemp())
+    out = {}
+    for window, ex_len in DATASET_CASES:
+        ref = ref_dataset.SGDataset(ddef, dproc, window, "example", ex_len)
+        rs = np.random.RandomState(window)
+        idx = np.array(list(rs.randint(0, len(ref), size=40)) + [0, len(ref) - 1], dtype=np.int64)
+        tag = f"w{window}_ex{ex_len}"
+        out[tag + "_len"] = len(ref)
+        out[tag + "_idx"] = idx
+        out[tag + "_R"] = ref.R[idx].numpy()
+        out[tag + "_S"] = ref.S[idx].numpy()
+        out[tag + "_digest"] = np.array([[fx.digest(t.numpy()) for t in ref[int(i)]] for i in idx])
+    out["label_w64_L"] = ref_dataset.SGDataset(ddef, dproc, 64, "label", 128).L.numpy()
+    np.savez_compressed(os.path.join(GOLD, "dataset_windows.npz"), **out)
+    print("dataset_windows golden written")
+
+
+ANIM_KEYS = ["root_pos", "root_rot", "root_vel", "root_vrt", "lpos", "lrot", "ltxy", "lvel", "lvrt", "cpos", "crot", "ctxy", "cvel",
+             "cvrt", "gaze_pos", "gaze_dir"]
+ANIM_CUTS = {"full": None, "cut10_80": (10, 80)}
+ANIM_SAMPLES = 128        # values kept per preprocess_animation output: a fixed seeded sample of its flat indices
+
+
+def anim_sample_index(size, key):
+    return np.random.RandomState(sum(map(ord, key))).randint(0, size, size=min(ANIM_SAMPLES, size))
+
+
+def write_animation_io_golden():
+    """The reference's BVH writer (anim/bvh.py:137) on seeded channels: the file it writes, byte for byte; its BVH loader
+    (anim/bvh.py:4) and preprocess_animation (data_pipeline.py:90) on the 120-frame synthetic clip of tests/_fixtures.py:
+    fingerprints of what the loader returns and, per preprocess_animation output, its shape, max |value| and a seeded sample."""
+    import copy
+    import tempfile
+    from tests import _fixtures as fx
+    ref_shim.install()
+    from anim import bvh
+    from data_pipeline import preprocess_animation as ref_pa
+    tmp = tempfile.mkdtemp()
+    d = fx.skeleton()
+    rs = np.random.RandomState(0)
+    pos = rs.randn(5, 75, 3).astype(np.float32); rot = (rs.randn(5, 75, 3) * 50).astype(np.float32)
+    bvh.save(os.path.join(tmp, "a.bvh"), dict(order="zyx", offsets=pos[0], names=d["bone_names"], frametime=d["dt"],
+                                              parents=np.array(d["parents"]), positions=pos, rotations=rot))
+    with open(os.path.join(tmp, "a.bvh"), "rb") as f:
+        out = {"writer_bvh": np.frombuffer(f.read(), dtype=np.uint8)}
+    a_ref = bvh.load(fx.make_synthetic_bvh(os.path.join(tmp, "s.bvh"), frames=120))
+    for k in ("rotations", "positions", "offsets", "parents"):
+        out["load_" + k] = fx.digest(np.asarray(a_ref[k], dtype=np.float64))
+    for tag, cut in ANIM_CUTS.items():
+        ar = copy.deepcopy(a_ref)
+        if cut:
+            ar["rotations"], ar["positions"] = ar["rotations"][cut[0]:cut[1]], ar["positions"][cut[0]:cut[1]]
+        for k, v in zip(ANIM_KEYS, ref_pa(ar)):
+            v = np.asarray(v)
+            out[f"{tag}_{k}_shape"] = np.array(v.shape)
+            out[f"{tag}_{k}_absmax"] = np.float64(np.abs(v).max())
+            out[f"{tag}_{k}_sample"] = v.reshape(-1)[anim_sample_index(v.size, k)]
+    np.savez_compressed(os.path.join(GOLD, "animation_io.npz"), **out)
+    print("animation_io golden written")
+
+
+PICKLE_SIZES = dict(speech=(81, 8, 8), decoder=(1134, 1131, 8, 8, 16, 2), style=(1134, 16, 4))
+
+
+def write_pickles_golden():
+    """Whole-module pickles (torch.save of the module, as the reference's train.py saves its networks) of small instances of the
+    reference's SpeechEncoder, Decoder and StyleEncoder, stored as the bytes of each file.  Only their layout matters to the test
+    that loads them, so to keep them small every parameter is zero and the positional-encoding table the reference keeps as a
+    plain attribute (20000 x embed_dim) is cut to its first 16 rows; zeggs_b200 recomputes that table."""
+    import io
+    m = ref_shim.ref_modules()
+    sty = m.StyleEncoder(*PICKLE_SIZES["style"], type="attn", use_vae=True)
+    sty.encoder.pos_enc.pos_enc = sty.encoder.pos_enc.pos_enc[:16].clone()
+    out = {}
+    for name, net in (("speech_encoder", m.SpeechEncoder(*PICKLE_SIZES["speech"])), ("decoder", m.Decoder(*PICKLE_SIZES["decoder"])),
+                      ("style_encoder", sty)):
+        with torch.no_grad():
+            for p in net.parameters():
+                p.zero_()
+        buf = io.BytesIO()
+        torch.save(net, buf)
+        out[name] = np.frombuffer(buf.getvalue(), dtype=np.uint8)
+    np.savez_compressed(os.path.join(GOLD, "pickles.npz"), **out)
+    print("pickles golden written")
+
+
 def write_pose_post_golden(T=40):
     """generate.py:389-406 + utils.write_bvh through the reference's own functions: what bvh.save receives for a synthetic clip."""
     ref_shim.install()
@@ -328,6 +438,10 @@ def write_pose_post_golden(T=40):
         rutils.bvh.save = orig
     np.savez_compressed(os.path.join(GOLD, "pose_post.npz"), **out)
     print("pose_post golden written")
+
+
+REFERENCE_IO = dict(mel_clip=write_mel_clip_golden, dataset=write_dataset_golden, animation_io=write_animation_io_golden,
+                    pickles=write_pickles_golden)
 
 
 if __name__ == "__main__":

@@ -32,6 +32,38 @@ def make_synthetic_bvh(path, frames=420, seed=31):
     return path
 
 
+def write_processed_data(d):
+    """A 900-frame processed_data.npz with the reference's schema (data_pipeline.py:650-684) plus its data_definition.json, in
+    directory `d`; the 120-frame middle range is short enough to exercise the style-example clamping and tail repetition."""
+    from zeggs_b200 import synth
+    from zeggs_b200.data import KEYS
+    st = synth.load_stats()
+    rs = np.random.RandomState(3)
+    N = 900
+    data = {"X_audio_features": rs.randn(N, 81).astype(np.float32)}
+    win = synth.make_pose_windows(1, N, seed=4)
+    for k in KEYS:
+        data["Y_" + k] = win[k][0]
+    ranges = np.array([[0, 300], [300, 420], [420, 900]], dtype=np.int64)
+    data.update(ranges_train=ranges, ranges_valid=ranges[:1], ranges_train_labels=np.array([0, 2, 1]),
+                ranges_valid_labels=np.array([0]))
+    for k in ("audio_input_mean", "audio_input_std", "anim_input_mean", "anim_input_std", "anim_output_mean", "anim_output_std"):
+        data[k] = st[k]
+    np.savez(os.path.join(d, "processed_data.npz"), **data)
+    details = dict(bone_names=[f"b{i}" for i in range(75)], label_names=["Neutral", "Happy", "Sad"],
+                   parents=[int(p) for p in st["parents"]], dt=float(st["dt"]))
+    with open(os.path.join(d, "data_definition.json"), "w") as f:
+        json.dump(details, f)
+    return os.path.join(d, "data_definition.json"), os.path.join(d, "processed_data.npz")
+
+
+def digest(x):
+    """16-byte fingerprint (uint8[16]) of an array's dtype, shape and bytes: equal fingerprints <=> bit-identical arrays."""
+    import hashlib
+    a = np.ascontiguousarray(np.asarray(x))
+    return np.frombuffer(hashlib.sha256(f"{a.dtype.str}{a.shape}".encode() + a.tobytes()).digest()[:16], dtype=np.uint8)
+
+
 def make_wav(path, seconds=4.0, seed=32):
     from scipy.io import wavfile
     from zeggs_b200 import synth

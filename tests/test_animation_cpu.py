@@ -1,16 +1,12 @@
-"""Host-side data-format edges of generate_gesture (CPU): BVH parse / feature extraction / BVH write of this package against the
-reference's own functions (when /root/reference is importable, i.e. in the dev container) and against the committed goldens."""
-import copy
+"""Host-side data-format edges of generate_gesture (CPU): BVH parse / feature extraction / BVH write of this package against what
+the reference's own functions returned for the same inputs (tests/golden/animation_io.npz and pose_post.npz, oracle/make_golden.py)."""
 import os
 
 import numpy as np
-import pytest
 
-from oracle import pose_oracle as po, ref_shim
+from oracle import make_golden as mg, pose_oracle as po
 from tests import _fixtures as fx
 from zeggs_b200 import animation, bvhio, generate
-
-needs_ref = pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
 
 
 def test_pose_oracle_matches_reference_golden(golden_dir):
@@ -38,35 +34,26 @@ def test_bvh_round_trip(tmp_path):
     assert list(a["parents"]) == list(b["parents"]) and a["names"] == b["names"]
 
 
-@needs_ref
-def test_bvh_writer_is_byte_identical_to_the_reference_writer(tmp_path):
-    ref_shim.install()
-    from anim import bvh
+def test_bvh_writer_is_byte_identical_to_the_reference_writer(tmp_path, golden_dir):
+    ref = np.load(os.path.join(golden_dir, "animation_io.npz"))["writer_bvh"].tobytes()
     d = fx.skeleton()
     rs = np.random.RandomState(0)
     pos = rs.randn(5, 75, 3).astype(np.float32); rot = (rs.randn(5, 75, 3) * 50).astype(np.float32)
-    bvh.save(str(tmp_path / "a.bvh"), dict(order="zyx", offsets=pos[0], names=d["bone_names"], frametime=d["dt"],
-                                           parents=np.array(d["parents"]), positions=pos, rotations=rot))
     bvhio.save_bvh(str(tmp_path / "b.bvh"), pos, rot, d["parents"], d["bone_names"], "zyx", d["dt"])
-    assert open(tmp_path / "a.bvh").read() == open(tmp_path / "b.bvh").read()
+    assert open(tmp_path / "b.bvh", "rb").read() == ref
 
 
-@needs_ref
-def test_load_and_preprocess_animation_match_the_reference(tmp_path):
-    ref_shim.install()
-    from anim import bvh
-    from data_pipeline import preprocess_animation as ref_pa
+def test_load_and_preprocess_animation_match_the_reference(tmp_path, golden_dir):
+    g = np.load(os.path.join(golden_dir, "animation_io.npz"))
     p = fx.make_synthetic_bvh(str(tmp_path / "s.bvh"), frames=120)
-    a_ref, a = bvh.load(p), animation.load_bvh(p)
+    a = animation.load_bvh(p)
     for k in ("rotations", "positions", "offsets", "parents"):
-        assert np.abs(np.asarray(a_ref[k], dtype=np.float64) - np.asarray(a[k], dtype=np.float64)).max() == 0.0
-    keys = ["root_pos", "root_rot", "root_vel", "root_vrt", "lpos", "lrot", "ltxy", "lvel", "lvrt", "cpos", "crot", "ctxy", "cvel",
-            "cvrt", "gaze_pos", "gaze_dir"]
-    for cut in (None, (10, 80)):
-        ar = copy.deepcopy(a_ref)
-        if cut:
-            ar["rotations"], ar["positions"] = ar["rotations"][cut[0]:cut[1]], ar["positions"][cut[0]:cut[1]]
-        R = dict(zip(keys, ref_pa(ar)))
+        assert np.array_equal(fx.digest(np.asarray(a[k], dtype=np.float64)), g["load_" + k]), k
+    for tag, cut in mg.ANIM_CUTS.items():
         O = animation.preprocess_animation(animation.trim(a, cut))
+        assert set(O) <= set(mg.ANIM_KEYS)
         for k, v in O.items():
-            assert np.abs(R[k].astype(np.float64) - v).max() <= 1e-5 * max(1.0, np.abs(R[k]).max()), k
+            assert v.shape == tuple(g[f"{tag}_{k}_shape"]), (tag, k)
+            ref = g[f"{tag}_{k}_sample"].astype(np.float64)
+            got = v.reshape(-1)[mg.anim_sample_index(v.size, k)]
+            assert np.abs(ref - got).max() <= 1e-5 * max(1.0, float(g[f"{tag}_{k}_absmax"])), (tag, k)

@@ -1,69 +1,53 @@
-"""Window supplier (zeggs_b200.data.WindowDataset) against the LIVE reference dataset (ZEGGS/dataset.py:9-204) on a synthetic
+"""Window supplier (zeggs_b200.data.WindowDataset) against the reference dataset (ZEGGS/dataset.py:9-204) on a synthetic
 processed_data.npz with the reference's schema (data_pipeline.py:650-684): same sliding windows, same style-example windows
-(edge clamping, tail repetition), same one-hot labels.  Skipped where the reference tree is absent (the GPU box)."""
-import json
+(edge clamping, tail repetition), same one-hot labels.  What the reference returned is stored in tests/golden/dataset_windows.npz
+(oracle/make_golden.py dataset): window rows and range indices as they are, every returned tensor as a fingerprint of its bytes."""
+import os
 
 import numpy as np
 import pytest
 import torch
 
-from oracle import ref_shim
-from zeggs_b200 import synth
+from tests import _fixtures as fx
 from zeggs_b200.data import KEYS, WindowDataset
-
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
 
 
 @pytest.fixture(scope="module")
 def files(tmp_path_factory):
-    d = tmp_path_factory.mktemp("ds")
-    st = synth.load_stats()
-    rs = np.random.RandomState(3)
-    N = 900
-    data = {"X_audio_features": rs.randn(N, 81).astype(np.float32)}
-    win = synth.make_pose_windows(1, N, seed=4)
-    for k in KEYS:
-        data["Y_" + k] = win[k][0]
-    ranges = np.array([[0, 300], [300, 420], [420, 900]], dtype=np.int64)       # a short range exercises the clamping
-    data.update(ranges_train=ranges, ranges_valid=ranges[:1], ranges_train_labels=np.array([0, 2, 1]),
-                ranges_valid_labels=np.array([0]))
-    for k in ("audio_input_mean", "audio_input_std", "anim_input_mean", "anim_input_std", "anim_output_mean", "anim_output_std"):
-        data[k] = st[k]
-    np.savez(d / "processed_data.npz", **data)
-    details = dict(bone_names=[f"b{i}" for i in range(75)], label_names=["Neutral", "Happy", "Sad"],
-                   parents=[int(p) for p in st["parents"]], dt=float(st["dt"]))
-    with open(d / "data_definition.json", "w") as f:
-        json.dump(details, f)
-    return d / "data_definition.json", d / "processed_data.npz"
+    return fx.write_processed_data(str(tmp_path_factory.mktemp("ds")))
+
+
+@pytest.fixture(scope="module")
+def golden(golden_dir):
+    return np.load(os.path.join(golden_dir, "dataset_windows.npz"))
 
 
 @pytest.mark.parametrize("window,ex_len", [(64, 128), (100, 256), (64, 64)])
-def test_windows_and_examples_match_reference(files, window, ex_len):
-    ref_shim.install()
-    import dataset as ref_dataset
+def test_windows_and_examples_match_reference(files, golden, window, ex_len):
     ddef, dproc = files
-    ref = ref_dataset.SGDataset(ddef, dproc, window, "example", ex_len)
+    tag = f"w{window}_ex{ex_len}"
     ours = WindowDataset(ddef, dproc, window, "example", ex_len, seed=0)
-    assert len(ours) == len(ref)
+    assert len(ours) == int(golden[tag + "_len"])
     rs = np.random.RandomState(window)
-    for i in list(rs.randint(0, len(ref), size=40)) + [0, len(ref) - 1]:
-        item = ref[int(i)]
+    idx = list(rs.randint(0, len(ours), size=40)) + [0, len(ours) - 1]
+    assert np.array_equal(idx, golden[tag + "_idx"])
+    for j, i in enumerate(idx):
+        ref_rows, ref_digest = golden[tag + "_R"][j], golden[tag + "_digest"][j]
         start, ri = int(ours.starts[i]), int(ours.rng_idx[i])
         rows = torch.arange(start, start + window)
-        assert torch.equal(rows, ref.R[int(i)]) and ri == int(ref.S[int(i)])
-        assert torch.equal(ours.X[rows], item[0])
-        for j, k in enumerate(KEYS):
-            assert torch.equal(ours.Y[k][rows], item[1 + j]), k
+        assert np.array_equal(rows.numpy(), ref_rows) and ri == int(golden[tag + "_S"][j])
+        assert np.array_equal(fx.digest(ours.X[rows].numpy()), ref_digest[0])
+        for k, key in enumerate(KEYS):
+            assert np.array_equal(fx.digest(ours.Y[key][rows].numpy()), ref_digest[1 + k]), key
         ex = ours._example(start, ri)
-        assert ex.shape == item[10].shape and torch.equal(ex, item[10])
+        assert np.array_equal(fx.digest(ex.numpy()), ref_digest[10])
 
 
-def test_label_batches_and_host_batches(files):
-    ref_shim.install()
-    import dataset as ref_dataset
+def test_label_batches_and_host_batches(files, golden):
     ddef, dproc = files
-    ref = ref_dataset.SGDataset(ddef, dproc, 64, "label", 128)
+    ref_L = torch.from_numpy(golden["label_w64_L"])
     ours = WindowDataset(ddef, dproc, 64, "label", 128, seed=5)
+    assert len(ours) == len(ref_L)
     b = ours.sample_host_batch(6)
     assert b["style"].shape == (6, 3) and torch.all(b["style"].sum(1) == 1)
     assert b["audio"].shape == (6, 64, 81) and b["lpos"].shape == (6, 64, 75, 3)
@@ -71,4 +55,4 @@ def test_label_batches_and_host_batches(files):
     ours2 = WindowDataset(ddef, dproc, 64, "label", 128, seed=5)
     idx = ours2.rs.randint(0, len(ours2.starts), size=6)
     for r, i in enumerate(idx):
-        assert torch.equal(b["style"][r], ref.L[int(i)])
+        assert torch.equal(b["style"][r], ref_L[int(i)])

@@ -2,10 +2,8 @@
 and the reference's whole-module pickles un-pickle into zeggs_b200.modules classes when it is registered as `modules`."""
 import sys
 
-import pytest
 import torch
 
-from oracle import ref_shim
 from zeggs_b200 import modules, synth
 
 
@@ -24,25 +22,29 @@ def test_state_dict_keys_and_shapes_match_reference_layout():
     assert (d.hidden_size, d.speech_encoding_size, d.style_encoding_size) == (1024, 64, 64)
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
-def test_reference_pickles_unpickle_into_our_classes():
+def test_reference_pickles_unpickle_into_our_classes(golden_dir):
+    """Whole-module pickles written by the reference's own classes (tests/golden/pickles.npz, oracle/make_golden.py pickles; small
+    instances of the shipped checkpoints' classes) load as zeggs_b200.modules classes when it is registered as `modules`."""
+    import io
     import os
+    import numpy as np
+    from oracle.make_golden import PICKLE_SIZES
+    g = np.load(os.path.join(golden_dir, "pickles.npz"))
+    load = lambda name: torch.load(io.BytesIO(g[name].tobytes()), map_location="cpu", weights_only=False)
     saved = sys.modules.get("modules")
     sys.modules["modules"] = modules            # what INTEGRATION.md tells a maintainer to do
     try:
-        d = os.path.join(ref_shim.REF_ROOT, "data", "outputs", "v1", "saved_models")
-        dec = torch.load(os.path.join(d, "decoder.pt"), map_location="cpu", weights_only=False)
-        enc = torch.load(os.path.join(d, "speech_encoder.pt"), map_location="cpu", weights_only=False)
-        sty = torch.load(os.path.join(d, "style_encoder.pt"), map_location="cpu", weights_only=False)
+        dec, enc, sty = load("decoder"), load("speech_encoder"), load("style_encoder")
     finally:
         if saved is not None:
             sys.modules["modules"] = saved
         else:
             del sys.modules["modules"]
     assert type(dec) is modules.Decoder and type(enc) is modules.SpeechEncoder and type(sty) is modules.StyleEncoder
-    assert (dec.hidden_size, dec.speech_encoding_size, dec.style_encoding_size) == (1024, 64, 64)
+    _, _, S, Z, H, _ = PICKLE_SIZES["decoder"]
+    assert (dec.hidden_size, dec.speech_encoding_size, dec.style_encoding_size) == (H, S, Z)
     assert len(dec._weights()) == 18 and len(enc._weights()) == 6 and len(sty._weights()) == 20
-    assert sty.encoder.pos_enc.table(5).shape == (5, 128)
+    assert sty.encoder.pos_enc.table(5).shape == (5, 2 * PICKLE_SIZES["style"][2])
 
 
 def test_lane_context_is_scoped_and_nestable():

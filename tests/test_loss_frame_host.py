@@ -4,7 +4,6 @@ autograd (train.py:277-421 restated in oracle/model_oracle.py).  No GPU involved
 import ctypes as C
 import os
 import subprocess
-import tempfile
 
 import numpy as np
 import pytest
@@ -23,8 +22,8 @@ GROUPS = [  # (start, n, term, w, dterm, dw)
 
 
 @pytest.fixture(scope="module")
-def harness():
-    out = os.path.join(tempfile.gettempdir(), "libzeggs_loss_host.so")
+def harness(tmp_path_factory):
+    out = str(tmp_path_factory.mktemp("host") / "libzeggs_loss_host.so")
     src = os.path.join(ROOT, "tests", "host", "loss_host.cu")
     r = subprocess.run(["/usr/local/cuda/bin/nvcc", "-O2", "-std=c++17", "-Xcompiler", "-fPIC", "-shared", "-o", out, src],
                        capture_output=True, text=True)

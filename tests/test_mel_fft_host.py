@@ -4,7 +4,6 @@ emulation of the warp's 32 x 25 decomposition and the two-real-frames separation
 import ctypes as C
 import os
 import subprocess
-import tempfile
 
 import numpy as np
 import pytest
@@ -13,8 +12,8 @@ from tests._util import ROOT
 
 
 @pytest.fixture(scope="module")
-def harness():
-    out = os.path.join(tempfile.gettempdir(), "libzeggs_mel_fft_host.so")
+def harness(tmp_path_factory):
+    out = str(tmp_path_factory.mktemp("host") / "libzeggs_mel_fft_host.so")
     src = os.path.join(ROOT, "tests", "host", "mel_fft_host.cu")
     r = subprocess.run(["/usr/local/cuda/bin/nvcc", "-O2", "-std=c++17", "--expt-relaxed-constexpr", "-Xcompiler", "-fPIC", "-shared",
                         "-o", out, src], capture_output=True, text=True)

@@ -1,5 +1,7 @@
-"""Pin the oracle against the LIVE reference (imported from /root/reference) with the shipped
-pretrained v1 weights.  Skipped where the reference tree is absent (the GPU box)."""
+"""Pin the oracle against the reference: against the live reference with the shipped pretrained v1 weights (skipped where the
+reference tree is absent), and against the reference's preprocess_audio output stored in tests/golden/mel_clip90.npz."""
+import os
+
 import numpy as np
 import pytest
 import torch
@@ -8,13 +10,13 @@ from oracle import model_oracle as mo
 from oracle import ref_shim
 from zeggs_b200 import synth
 
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
-
 NAMES = ["root_pos", "root_rot", "root_vel", "root_vrt", "lpos", "ltxy", "lvel", "lvrt"]
 
 
 @pytest.fixture(scope="module")
 def pretrained():
+    if not ref_shim.available():
+        pytest.skip("reference tree not present")
     nets = ref_shim.load_pretrained("v1")
     P = {}
     for pre, key in (("speech_encoder.", "speech_encoder"), ("style_encoder.", "style_encoder"), ("decoder.", "decoder")):
@@ -51,11 +53,12 @@ def test_pretrained_v1_forward(pretrained):
             assert torch.max(torch.abs(o - r)) <= tol, n
 
 
-def test_live_mel_matches(pretrained):
+def test_live_mel_matches(golden_dir):
+    """preprocess_audio of a 1.5 s clip at 60 fps / 90 frames against the reference's output (oracle/make_golden.py mel_clip)."""
     from oracle import mel_oracle
-    from oracle.make_golden import audio_params
-    pa = ref_shim.ref_preprocess_audio()
-    wav = synth.make_waveforms(1, 24000, seed=3)[0]
-    ref = pa(wav, 60, 90, audio_params(200), ["mel_spec", "energy"])
+    g = np.load(os.path.join(golden_dir, "mel_clip90.npz"))
+    wav = synth.make_waveforms(1, int(g["n_samples"]), seed=int(g["wav_seed"]))[0]
+    ref = g["feat"]
+    assert ref.shape == (90, 81)
     got = mel_oracle.preprocess_audio(wav, 60, 90)
     assert np.max(np.abs(ref - got)) <= 1e-6

@@ -171,6 +171,18 @@ void zeggs_debug_set_tc_cluster(int n); /* development aid: cap the thread-block
 int zeggs_debug_get_tc_cluster(void);   /* cluster size the last tc forward launch used */
 int zeggs_decoder_window_fwd(const zeggs_decoder_fwd_args* a, void* stream);
 
+/* Resumable window (streaming inference): zeggs_decoder_window_fwd with the GRU state of frame 0 taken from the caller and the
+ * state of frame T-1 handed back.  Frame 0 is still the given pose (pose0, root_pos0, root_rot0); only the state that frame 1
+ * starts from changes.  A continuation is a literal sub-window of the one-shot window: pass the pose, root and state of the last
+ * emitted frame and the speech / style / gaze rows from that frame onward.  s == NULL is zeggs_decoder_window_fwd.
+ * Inference only: save_for_backward must be 0.  With T == 1, h_final is the initial state. */
+typedef struct {
+  const float* h_init;          /* [2,B,H] GRU state (layer, sample, unit) = nn.GRU's h layout, as zeggs_decoder_step_args.h_in; NULL = CellStateEncoder */
+  const int* init_from_state;   /* [B] int32 device: 1 = sample b starts from h_init[:,b], 0 = from the CellStateEncoder; NULL with h_init set = all 1 */
+  float* h_final;               /* [2,B,H] state at frame T-1, or NULL */
+} zeggs_decoder_state_args;
+int zeggs_decoder_window_fwd_state(const zeggs_decoder_fwd_args* a, const zeggs_decoder_state_args* s, void* stream);
+
 /* Backward of zeggs_decoder_window_fwd (the autograd of modules.py:47-162: full BPTT through the GRU stack,
  * the pose feedback, the gaze transform and the root integration).  Needs the forward's workspace
  * (save_for_backward = 1) and outputs (Y, root_pos, root_rot) untouched.  Gradient buffers have the shapes
@@ -261,8 +273,8 @@ int zeggs_style_enc_bwd(const zeggs_style_enc_args* a, const zeggs_style_enc_gra
  * One teacher-forced decoder step (RecurrentDecoderNormal.forward, modules.py:179-185), fp32 throughout:
  *   pose [B,1134] (the normalised input vector of modules.py:699-713), speech [B,S], style [B,Z], h_in [2,B,H]
  *   -> y [B,1131] (normalised output of layer2), h_out [2,B,H].
- * The tight parity point (<= 1e-4 vs the reference per step) and the unit of streaming inference; windows go through
- * zeggs_decoder_window_fwd.
+ * The tight parity point (<= 1e-4 vs the reference per step); windows go through zeggs_decoder_window_fwd, streamed windows
+ * through zeggs_decoder_window_fwd_state.
  */
 typedef struct {
   int B, H, S, Z;

@@ -67,6 +67,11 @@ class DecoderBwdArgs(C.Structure):
         [("workspace_bytes", C.c_size_t), ("packed_bwd_tc", C.c_void_p), ("workspace_tc", C.c_void_p), ("phase", C.c_int)])
 
 
+class DecoderStateArgs(C.Structure):
+    """zeggs_decoder_state_args: GRU state in ([2,B,H], per-sample int32 selector) and out ([2,B,H]) of a resumable window."""
+    _fields_ = [("h_init", C.c_void_p), ("init_from_state", C.c_void_p), ("h_final", C.c_void_p)]
+
+
 def _struct(name, ints=(), floats=(), ptrs=(), tail=()):
     fields = [(n, C.c_int) for n in ints] + [(n, C.c_float) for n in floats] + [(n, C.c_void_p) for n in ptrs] + list(tail)
     return type(name, (C.Structure,), {"_fields_": fields})
@@ -101,7 +106,8 @@ def struct_mirrors():
     return {"zeggs_ctx": Ctx, "zeggs_mel_args": MelArgs, "zeggs_loudness_args": LoudnessArgs, "zeggs_decoder_fwd_args": DecoderFwdArgs,
             "zeggs_decoder_bwd_args": DecoderBwdArgs, "zeggs_speech_enc_args": SpeechEncArgs, "zeggs_speech_enc_grads": SpeechEncGrads,
             "zeggs_style_enc_args": StyleEncArgs, "zeggs_style_enc_grads": StyleEncGrads, "zeggs_decoder_step_args": DecoderStepArgs,
-            "zeggs_loss_args": LossArgs, "zeggs_pose_post_args": PosePostArgs, "zeggs_gather_args": GatherArgs}
+            "zeggs_loss_args": LossArgs, "zeggs_pose_post_args": PosePostArgs, "zeggs_gather_args": GatherArgs,
+            "zeggs_decoder_state_args": DecoderStateArgs}
 
 
 SYMBOLS = [
@@ -125,6 +131,7 @@ SYMBOLS = [
     ("zeggs_decoder_pack_weights", C.c_int, [C.POINTER(DecoderFwdArgs), C.c_void_p, C.c_void_p]),
     ("zeggs_decoder_workspace_bytes", C.c_size_t, [C.c_int] * 6),
     ("zeggs_decoder_window_fwd", C.c_int, [C.POINTER(DecoderFwdArgs), C.c_void_p]),
+    ("zeggs_decoder_window_fwd_state", C.c_int, [C.POINTER(DecoderFwdArgs), C.POINTER(DecoderStateArgs), C.c_void_p]),
     ("zeggs_decoder_packed_tc_bytes", C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     ("zeggs_decoder_tc_workspace_bytes", C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     ("zeggs_decoder_pack_weights_tc", C.c_int, [C.POINTER(DecoderFwdArgs), C.c_void_p, C.c_void_p]),

@@ -95,7 +95,7 @@ extern "C" size_t zeggs_struct_size(const char* name) {
 #define ZS(T) if (!strcmp(name, #T)) return sizeof(T);
   ZS(zeggs_ctx) ZS(zeggs_mel_args) ZS(zeggs_loudness_args) ZS(zeggs_decoder_fwd_args) ZS(zeggs_decoder_bwd_args) ZS(zeggs_speech_enc_args)
   ZS(zeggs_speech_enc_grads) ZS(zeggs_style_enc_args) ZS(zeggs_style_enc_grads) ZS(zeggs_decoder_step_args) ZS(zeggs_loss_args)
-  ZS(zeggs_pose_post_args) ZS(zeggs_gather_args)
+  ZS(zeggs_pose_post_args) ZS(zeggs_gather_args) ZS(zeggs_decoder_state_args)
 #undef ZS
   return 0;
 }

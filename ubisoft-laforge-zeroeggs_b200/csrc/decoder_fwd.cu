@@ -96,14 +96,26 @@ __global__ void decoder_prologue_kernel(zeggs_decoder_fwd_args a, DecGeom g, flo
   if (threadIdx.x < 4) a.root_rot[((size_t)b * T) * 4 + threadIdx.x] = a.root_rot0[b * 4 + threadIdx.x];
 }
 
-// cse_out[B][2H] -> H0[slot0], H1[slot0] in k-major [bt][H][32]   (modules.py:243)
-__global__ void cse_scatter_kernel(int B, int H, const float* __restrict__ cse_out, float* __restrict__ h0, float* __restrict__ h1) {
+// initial GRU state -> H0[slot0], H1[slot0] in k-major [bt][H][32].  Per sample b the source is the CellStateEncoder output
+// cse_out[B][2H] (modules.py:243) or, when h_init is set and from_state is NULL or from_state[b] != 0, the caller's h_init[2][B][H].
+__global__ void cse_scatter_kernel(int B, int H, const float* __restrict__ cse_out, const float* __restrict__ h_init,
+                                   const int* __restrict__ from_state, float* __restrict__ h0, float* __restrict__ h1) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= B * 2 * H) return;
   int b = i / (2 * H), r = i % (2 * H);
   int l = r / H, j = r % H;
+  const bool carry = h_init != nullptr && (from_state == nullptr || from_state[b] != 0);
   float* dst = l == 0 ? h0 : h1;
-  dst[((size_t)(b / 32) * H + j) * 32 + (b % 32)] = cse_out[i];
+  dst[((size_t)(b / 32) * H + j) * 32 + (b % 32)] = carry ? h_init[((size_t)l * B + b) * H + j] : cse_out[i];
+}
+
+// h0 / h1 of one time slot (k-major [bt][H][32]) -> out[2][B][H]
+__global__ void state_gather_kernel(int B, int H, const float* __restrict__ h0, const float* __restrict__ h1, float* __restrict__ out) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= 2 * B * H) return;
+  int l = i / (B * H), r = i % (B * H);
+  int b = r / H, j = r % H;
+  out[i] = (l == 0 ? h0 : h1)[((size_t)(b / 32) * H + j) * 32 + (b % 32)];
 }
 
 // S01[t][bt][n][32], n in [0,4H): n<H: b0[n] + W0[n, 1134:] . cond ; else b_ih0[n-H] + W_ih0[n-H, H+1134:] . cond
@@ -355,9 +367,13 @@ static int launch_fwd(const zeggs_decoder_fwd_args& a, const DecGeom& g, const D
   return ZEGGS_OK;
 }
 
-extern "C" int zeggs_decoder_window_fwd(const zeggs_decoder_fwd_args* ap, void* stream_) {
+// s == NULL: the window starts from the CellStateEncoder and no state is exported (zeggs_decoder_window_fwd)
+static int window_fwd(const zeggs_decoder_fwd_args* ap, const zeggs_decoder_state_args* s, void* stream_) {
   int rc = check_fwd_args(ap); if (rc) return rc;
   const zeggs_decoder_fwd_args& a = *ap;
+  const float* h_init = s ? s->h_init : nullptr;
+  const int* from_state = s ? s->init_from_state : nullptr;
+  float* h_final = s ? s->h_final : nullptr;
   CtxScope ctx_scope(a.ctx);
   cudaStream_t stream = (cudaStream_t)stream_;
   DecGeom g = make_geom(a.B, a.H, a.S, a.Z);
@@ -373,11 +389,13 @@ extern "C" int zeggs_decoder_window_fwd(const zeggs_decoder_fwd_args* ap, void* 
   decoder_prologue_kernel<<<a.B, 256, 0, stream>>>(a, g, w.cse_in, w.XP + (size_t)slot1 * g.nbt * K1P * 32);
   count_launch();
   ZCHECK_LAUNCH();
-  // CellStateEncoder (modules.py:238-243)
-  rc = gemm_f32_auto(0, a.B, a.H, P_IN + a.Z, w.cse_in, P_IN + a.Z, a.Wc0, P_IN + a.Z, a.bc0, w.cse_h1, a.H, 1, 0, stream); if (rc) return rc;
-  rc = gemm_f32_auto(0, a.B, a.H, a.H, w.cse_h1, a.H, a.Wc1, a.H, a.bc1, w.cse_h2, a.H, 1, 0, stream); if (rc) return rc;
-  rc = gemm_f32_auto(0, a.B, 2 * a.H, a.H, w.cse_h2, a.H, a.Wc2, a.H, a.bc2, w.cse_out, 2 * a.H, 0, 0, stream); if (rc) return rc;
-  cse_scatter_kernel<<<ceil_div(a.B * 2 * a.H, 256), 256, 0, stream>>>(a.B, a.H, w.cse_out, w.H0, w.H1);
+  // CellStateEncoder (modules.py:238-243), unless every sample starts from the caller's state
+  if (h_init == nullptr || from_state != nullptr) {
+    rc = gemm_f32_auto(0, a.B, a.H, P_IN + a.Z, w.cse_in, P_IN + a.Z, a.Wc0, P_IN + a.Z, a.bc0, w.cse_h1, a.H, 1, 0, stream); if (rc) return rc;
+    rc = gemm_f32_auto(0, a.B, a.H, a.H, w.cse_h1, a.H, a.Wc1, a.H, a.bc1, w.cse_h2, a.H, 1, 0, stream); if (rc) return rc;
+    rc = gemm_f32_auto(0, a.B, 2 * a.H, a.H, w.cse_h2, a.H, a.Wc2, a.H, a.bc2, w.cse_out, 2 * a.H, 0, 0, stream); if (rc) return rc;
+  }
+  cse_scatter_kernel<<<ceil_div(a.B * 2 * a.H, 256), 256, 0, stream>>>(a.B, a.H, w.cse_out, h_init, from_state, w.H0, w.H1);
   count_launch();
   ZCHECK_LAUNCH();
   if (a.T > 1) {
@@ -402,7 +420,24 @@ extern "C" int zeggs_decoder_window_fwd(const zeggs_decoder_fwd_args* ap, void* 
     }
     if (rc) return rc;
   }
+  if (h_final) {
+    // both engines leave frame t's state in slot (save ? t : t & 1) of H0 / H1; state carry runs without save, and with T == 1
+    // slot 0 still holds the initial state
+    const size_t slot = (size_t)((a.T - 1) & 1) * g.nbt * a.H * 32;
+    state_gather_kernel<<<ceil_div(2 * a.B * a.H, 256), 256, 0, stream>>>(a.B, a.H, w.H0 + slot, w.H1 + slot, h_final);
+    count_launch();
+    ZCHECK_LAUNCH();
+  }
   return ZEGGS_OK;
+}
+
+extern "C" int zeggs_decoder_window_fwd(const zeggs_decoder_fwd_args* a, void* stream) { return window_fwd(a, nullptr, stream); }
+
+extern "C" int zeggs_decoder_window_fwd_state(const zeggs_decoder_fwd_args* a, const zeggs_decoder_state_args* s, void* stream) {
+  ZCHECK_ARG(a != nullptr, "decoder: null args");
+  ZCHECK_ARG(a->save_for_backward == 0, "decoder state carry is inference only: save_for_backward must be 0");
+  ZCHECK_ARG(s == nullptr || s->init_from_state == nullptr || s->h_init != nullptr, "decoder: init_from_state given without h_init");
+  return window_fwd(a, s, stream);
 }
 
 }  // namespace zeggs

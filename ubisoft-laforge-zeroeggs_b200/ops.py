@@ -281,6 +281,52 @@ def decoder_window_forward(dec, root_pos0, root_rot0, pose0, gaze_pos, speech, s
     return Y, rp, rq, (a, keep, ws)
 
 
+def decoder_window_forward_state(dec, root_pos0, root_rot0, pose0, gaze_pos, speech, style, stats, dt, h_init=None,
+                                 init_from_state=None):
+    """Resumable inference window (zeggs_decoder_window_fwd_state) -> (Y [B,T,1131], root_pos, root_rot, h_final [2,B,H]).
+    h_init [2,B,H]: GRU state frame 1 starts from (None: the CellStateEncoder); init_from_state [B] int32: per-sample choice between
+    h_init (1) and the CellStateEncoder (0), None = all h_init.  On the tensor-core engine batches above 32 run as 32-sample tiles."""
+    dev = speech.device
+    if dev.type != "cuda":
+        raise _lib.ZeggsError("zeggs_b200.Decoder runs on CUDA tensors only (no CPU fallback)")
+    ensure_scratch(dev)
+    B, T = speech.shape[0], speech.shape[1]
+    if init_from_state is not None and h_init is None:
+        raise _lib.ZeggsError("init_from_state needs h_init")
+    if B > 32 and resolve_engine(dec.hidden_size, dec.speech_encoding_size, dec.style_encoding_size):
+        outs = [decoder_window_forward_state(
+            dec, root_pos0[i:i + 32], root_rot0[i:i + 32], pose0[i:i + 32], gaze_pos[i:i + 32], speech[i:i + 32], style[i:i + 32],
+            stats, dt, None if h_init is None else h_init[:, i:i + 32],
+            None if init_from_state is None else init_from_state[i:i + 32]) for i in range(0, B, 32)]
+        Y, rp, rq, hf = zip(*outs)
+        return torch.cat(Y, 0), torch.cat(rp, 0), torch.cat(rq, 0), torch.cat(hf, 1)
+    H = dec.hidden_size
+    tensors = dict(root_pos0=_f32c(root_pos0, dev).reshape(B, 3), root_rot0=_f32c(root_rot0, dev).reshape(B, 4),
+                   pose0=_f32c(pose0, dev).reshape(B, P_OUT), gaze_pos=_f32c(gaze_pos, dev).reshape(B, T, 3),
+                   speech=_f32c(speech, dev), style=_f32c(style, dev))
+    if tensors["style"].shape[:2] != (B, T):
+        raise _lib.ZeggsError("style_encoding must be [B,T,Z] (modules.py:119)")
+    Y = torch.empty((B, T, P_OUT), dtype=torch.float32, device=dev)
+    rp = torch.empty((B, T, 3), dtype=torch.float32, device=dev)
+    rq = torch.empty((B, T, 4), dtype=torch.float32, device=dev)
+    h_final = torch.empty((2, B, H), dtype=torch.float32, device=dev)
+    tensors.update(Y=Y, root_pos=rp, root_rot=rq)
+    a, keep, ws = _decoder_args(dec, B, T, dev, tensors, stats, dt, False)
+    s = _lib.DecoderStateArgs(h_final=h_final.data_ptr())
+    if h_init is not None:
+        h_init = _f32c(h_init, dev)
+        if tuple(h_init.shape) != (2, B, H):
+            raise _lib.ZeggsError(f"h_init must be [2,B,H] = [2,{B},{H}], got {tuple(h_init.shape)}")
+        s.h_init = h_init.data_ptr()
+    if init_from_state is not None:
+        init_from_state = init_from_state.to(device=dev, dtype=torch.int32).contiguous()
+        if tuple(init_from_state.shape) != (B,):
+            raise _lib.ZeggsError(f"init_from_state must be [B] = [{B}]")
+        s.init_from_state = init_from_state.data_ptr()
+    _lib.check(_lib.lib().zeggs_decoder_window_fwd_state(a, s, _lib.stream_ptr()), "zeggs_decoder_window_fwd_state")
+    return Y, rp, rq, h_final
+
+
 _DEC_GRAD_NAMES = ["dW0", "db0", "dW_ih0", "db_ih0", "dW_hh0", "db_hh0", "dW_ih1", "db_ih1", "dW_hh1", "db_hh1",
                    "dW2", "db2", "dWc0", "dbc0", "dWc1", "dbc1", "dWc2", "dbc2"]
 
